@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the MAPDN var_voltage_control env step (BASELINE.json metric: env-steps/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1]): case33 (33-bus feeder), 4096 env instances per GPU, Bowl
 voltage barrier, noise on, synthetic load/PV profiles and random actions (the reference's data
@@ -335,8 +335,29 @@ class Timer:
         return float(t.item())
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(env, out_dir):
+    """Writes what the last timed ``env.step`` handed its caller (reward, terminated, info, and the observations the step
+    left in ``env.obs``) as ``out_dir/<name>.npy``, float64 (terminated as 0/1). When the arrays exceed 64 MiB in all, a
+    fixed sample of env rows (seed 0, sorted) is written instead, with their ids in ``env_ids.npy``."""
+    out = dict(reward=env.reward, terminated=env.terminated, info=env.info, obs=env.obs)
+    out = {k: v.cpu().numpy().astype(np.float64) for k, v in out.items()}
+    B = env.count
+    if sum(a.nbytes for a in out.values()) > DUMP_LIMIT_BYTES:
+        row = sum(a.nbytes for a in out.values()) // B + 8          # + its env id
+        keep = max(1, (DUMP_LIMIT_BYTES - (64 << 10)) // row)       # 64 KiB for the .npy headers
+        ids = np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+        out = {k: a[ids] for k, a in out.items()}
+        out["env_ids"] = (ids + env.offset).astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+
+
 def measure(sc, barrier, global_batch, K, W, Ke, tm, local, rank, flush, lanes=0, clocks=None, obs_dtypes=("f64",),
-            min_warm=0):
+            min_warm=0, dump_dir=None):
     """Device-timed and end-to-end throughput of one configuration, sharded over the ranks of this job."""
     import torch
     from mapdn_b200 import cases
@@ -389,6 +410,8 @@ def measure(sc, barrier, global_batch, K, W, Ke, tm, local, rank, flush, lanes=0
     launches = env.launch_count - launches0
     clk = clocks.stop(w0, w1, t_load0) if clocks is not None else None
     dev_ms = tm.max_over_ranks(sum(a.elapsed_time(b) for a, b in zip(ev0, ev1)))
+    if dump_dir is not None:
+        dump_outputs(env, dump_dir)
     assert returns.shape[0] == global_batch and bool(torch.isfinite(returns).all())
     # side metrics of the last timed step (SURVEY §8d): Newton iterations per solve, diverged fraction
     iters = env.get_field("nr_iters")[:, 0]
@@ -586,7 +609,8 @@ def run_ours(args):
         parity = parity_check(sc, barrier, B, local)
     clocks = ClockSampler(local) if rank == 0 else None
     m = measure(sc, barrier, B * world, K, W, Ke, tm, local, rank, flush, lanes=args.lanes, clocks=clocks,
-                obs_dtypes=("f64", "f32", "staged", "compact_f64", "compact_f32", "compact_zc_f64"), min_warm=50)
+                obs_dtypes=("f64", "f32", "staged", "compact_f64", "compact_f32", "compact_zc_f64"), min_warm=50,
+                dump_dir=args.dump_outputs if rank == 0 else None)
 
     # ---- the other BASELINE.json configurations of this GPU count ----
     subs = []
@@ -689,7 +713,13 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=0)
     ap.add_argument("--cpu-cores", type=int, default=0)
     ap.add_argument("--e2e-steps", type=int, default=50)
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step returned (rank 0's envs) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if args.warmup < 3:
         args.warmup = 3
     return run_reference(args) if args.impl == "reference" else run_ours(args)

@@ -87,3 +87,39 @@ def test_reference_fixture_leg_of_the_parity_record():
         rec = bench.reference_fixture_check(0, name=name, make_env=Standin)
         assert rec["n_steps"] >= 6 and rec["max_abs_dreward"] < 1e-11 and rec["max_abs_dinfo"] < 1e-11
         assert rec["max_abs_dobs"] < 1e-11 and rec["max_abs_dstate"] < 1e-9
+
+
+def test_dump_outputs_writes_what_the_step_returned(tmp_path):
+    """--dump-outputs: the last step's reward / terminated / info / obs as float64 .npy; past 64 MiB a fixed, seeded sample
+    of env rows (the same rows in every array) with their global env ids."""
+    import numpy as np
+    import torch
+    bench = _bench()
+
+    class Standin:
+        def __init__(self, B, obs_dim, offset=0):
+            g = torch.Generator().manual_seed(B)
+            self.count, self.offset = B, offset
+            self.reward = torch.rand(B, dtype=torch.float64, generator=g)
+            self.terminated = (torch.rand(B, generator=g) < 0.5).to(torch.uint8)
+            self.info = torch.rand(B, 11, dtype=torch.float64, generator=g)
+            self.obs = torch.rand(B, 6, obs_dim, dtype=torch.float64, generator=g)
+
+    env = Standin(64, 5)
+    bench.dump_outputs(env, str(tmp_path / "small"))
+    names = sorted(p.name for p in (tmp_path / "small").iterdir())
+    assert names == ["info.npy", "obs.npy", "reward.npy", "terminated.npy"]
+    for k in ("reward", "terminated", "info", "obs"):
+        a = np.load(tmp_path / "small" / f"{k}.npy")
+        assert a.dtype == np.float64 and np.array_equal(a, getattr(env, k).numpy().astype(np.float64))
+
+    big = Standin(4096, 400, offset=4096)                          # 4096 x (1 + 1 + 11 + 2400) fp64 = 75 MiB
+    for d in ("a", "b"):
+        bench.dump_outputs(big, str(tmp_path / d))
+    total = sum(p.stat().st_size for p in (tmp_path / "a").iterdir())
+    assert total <= 64 << 20
+    ids = np.load(tmp_path / "a" / "env_ids.npy").astype(np.int64) - big.offset
+    assert np.array_equal(ids, np.load(tmp_path / "b" / "env_ids.npy").astype(np.int64) - big.offset)
+    assert np.all(np.diff(ids) > 0) and len(ids) > 3000
+    assert np.array_equal(np.load(tmp_path / "a" / "obs.npy"), big.obs.numpy()[ids])
+    assert np.array_equal(np.load(tmp_path / "a" / "reward.npy"), big.reward.numpy()[ids])

@@ -1,18 +1,21 @@
-"""The batched runner feeds the REFERENCE's own learner code (models/maddpg.py, utilities/trainer.py) unchanged.
+"""The batched runner holds the conversation the REFERENCE's learners (models/*.py, utilities/trainer.py) expect.
 
-Runs where /root/reference exists (this container; it is imported in the test only, never by the product) on a CPU
-stand-in for BatchedVoltageControl; skipped on the GPU box. The GPU leg with the real env and an in-repo model of the
-same interface is tests/test_gpu_extras.py::test_marl_runner_on_device."""
-import os
-import sys
-from collections import namedtuple
+tests/golden/ref_learner_*.npz record the reference learners' side of that conversation, written by
+scripts/make_reference_extra_golden.py from the reference's own code: every get_actions / value / init_hidden call with a
+fingerprint of its inputs and its outputs, the batch shapes the reference's optimisation steps received, and, for the
+reference's own Model.train_process / Model.evaluation, the transitions and statistics it produced. Here a
+:class:`RecordedLearner` replays that side: each call checks that the runner passes what the reference learner was
+given and answers what the reference learner answered."""
+import json
+import types
 
 import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "models")), reason="reference tree not present")
+from conftest import ROOT
+
+GOLDEN = ROOT + "/tests/golden"
 
 
 class FakeBatchedEnv:
@@ -45,61 +48,106 @@ class FakeBatchedEnv:
         return reward, done, info
 
 
-@pytest.fixture
-def reference_on_path():
-    """The reference imports its agents lazily (models/model.py:150-163) from namespace packages (no __init__.py); an
-    unrelated `agents` distribution in site-packages would shadow them, so the reference's directories are registered
-    as the packages for the duration of the test."""
-    import types
-    saved = {k: sys.modules.get(k) for k in ("agents", "critics", "models", "utilities")}
-    for k in saved:
-        for name in [m for m in sys.modules if m == k or m.startswith(k + ".")]:
-            del sys.modules[name]
-        pkg = types.ModuleType(k)
-        pkg.__path__ = [os.path.join(REF, k)]
-        sys.modules[k] = pkg
-    sys.path.append(REF)
-    yield
-    sys.path.remove(REF)
-    for k, v in saved.items():
-        for name in [m for m in sys.modules if m == k or m.startswith(k + ".")]:
-            del sys.modules[name]
-        if v is not None:
-            sys.modules[k] = v
+class RecordedLearner:
+    """The recorded reference learner: same interface as the reference's models (get_actions, value,
+    policy_dicts[0].init_hidden, args, unpack_data)."""
+
+    def __init__(self, path, tol=1e-5):
+        g = np.load(path)
+        self.g, self.tol, self.k = g, tol, 0
+        self.calls = json.loads(str(g["calls"]))
+        data = g["data"]
+        self.a = {k: data[o:o + int(np.prod(shape))].reshape(shape) for k, (o, shape) in json.loads(str(g["index"])).items()}
+        self.args = types.SimpleNamespace(**json.loads(str(g["args"])))
+        self.policy_dicts = [types.SimpleNamespace(init_hidden=self.init_hidden)]
+
+    def _take(self, kind):
+        k = self.k
+        assert k < len(self.calls) and self.calls[k]["kind"] == kind, (k, kind)
+        self.k += 1
+        return k, self.calls[k]
+
+    def _check(self, k, name, t):
+        fp = self.a[f"c{k}_{name}"]
+        nd = len(fp) - 2
+        x = t.detach().double()
+        assert list(t.shape) == fp[:nd].astype(int).tolist(), (k, name)
+        for got, want in ((float(x.sum()), fp[nd]), (float((x * x).sum()), fp[nd + 1])):
+            assert abs(got - want) <= self.tol * (1.0 + abs(want)), (k, name, got, want)
+
+    def _out(self, k, name):
+        return torch.tensor(self.a[f"c{k}_{name}"], dtype=torch.float32)
+
+    def init_hidden(self):
+        k, _ = self._take("init_hidden")
+        return self._out(k, "hid")
+
+    def get_actions(self, state, status, exploration, actions_avail, target, last_hid):
+        k, c = self._take("get_actions")
+        assert c["status"] == status and c["exploration"] == bool(exploration) and target is False
+        self._check(k, "state", state)
+        self._check(k, "last_hid", last_hid)
+        lp = self._out(k, "log_prob_a") if c["log_prob"] else None
+        return self._out(k, "action"), self._out(k, "action_pol"), lp, None, self._out(k, "hid")
+
+    def value(self, obs, act):
+        k, _ = self._take("value")
+        self._check(k, "obs", obs)
+        self._check(k, "act", act)
+        return self._out(k, "value")
+
+    def unpack_data(self, batch):
+        raise TypeError("the recorded learner only consumes device batches")
+
+    def done(self):
+        return self.k == len(self.calls)
 
 
-def _reference_maddpg(n_agents, obs_dim, max_steps):
-    import yaml
-    from models.maddpg import MADDPG
-    from utilities.trainer import PGTrainer
-    d = yaml.safe_load(open(os.path.join(REF, "args", "default.yaml")))
-    d.update(yaml.safe_load(open(os.path.join(REF, "args", "alg_args", "maddpg.yaml")))["alg_args"])
-    d.update(agent_num=n_agents, obs_size=obs_dim, action_dim=1, cuda=False, max_steps=max_steps, action_scale=0.8,
-             action_bias=0.0, batch_size=8)
-    args = namedtuple("Args", d.keys())(**d)
-    trainer = PGTrainer(args, MADDPG, env=None, logger=None)
-    return args, trainer
-
-
-def test_reference_maddpg_learns_from_device_batches(reference_on_path):
-    from mapdn_b200.marl_runner import BatchedMarlRunner, DeviceTransitionBuffer, attach
+def _run_on_device_batches(alg):
+    """The runner collects through the (recorded) reference learner on the CPU stand-in env; at every lock-step the update
+    hook draws a device batch (same seeded generator as the recording) and hands it through attach(). Every field of every
+    batch has the shape, dtype, device, sum and sum of squares of the batch the reference's own value / policy / mixer
+    optimisation steps consumed and learned from when the recording was made."""
+    from mapdn_b200.marl_runner import BatchedMarlRunner, DeviceTransitionBuffer, TRANSITION_FIELDS, attach
     B, n, od, T = 5, 3, 7, 6
-    args, trainer = _reference_maddpg(n, od, max_steps=T)
-    net = attach(trainer.behaviour_net)
+    learner = RecordedLearner(f"{GOLDEN}/ref_learner_device_batches_{alg}.npz")
+    args = learner.args
+    assert args.max_steps == T
+    net = attach(learner)
     env = FakeBatchedEnv(B, n, od, episode_limit=4)
     buf = DeviceTransitionBuffer(32, B, n, od, act_dim=1, hid_dim=args.hid_size, device=env.device)
-    updates = []
+    gen = torch.Generator(device=env.device).manual_seed(17)          # BATCH_SEED of the recording script
+    want_fields = json.loads(str(learner.g["update_fields"]))
+    want_fp = learner.a["update_fingerprints"]
+    lock_steps, n_batches = [], [0]
 
-    def update(runner, stat):                      # the reference's own optimisation steps on a device batch
+    def update(runner, stat):                      # where the reference's own optimisation steps ran on a device batch
+        lock_steps.append(runner.steps // B)
         if len(runner.buffer) >= 2 * args.batch_size:
-            batch = runner.buffer.get_batch(args.batch_size, n_windows=2)
-            w0 = [p.detach().clone() for p in trainer.behaviour_net.value_dicts.parameters()]
-            trainer.value_transition_process(stat, batch)
-            trainer.policy_transition_process(stat, batch)
-            updates.append(any(not torch.equal(a, b) for a, b in
-                               zip(w0, trainer.behaviour_net.value_dicts.parameters())))
+            u = n_batches[0]
+            n_batches[0] += 1
+            batch = runner.buffer.get_batch(args.batch_size, n_windows=2, generator=gen)
+            got = net.unpack_data(batch)
+            assert len(got) == len(TRANSITION_FIELDS) == len(want_fields[u])
+            for f, t, (shape, dtype, device), (s1, s2) in zip(TRANSITION_FIELDS, got, want_fields[u], want_fp[u]):
+                assert [list(t.shape), str(t.dtype), t.device.type] == [shape, dtype, device], (u, f)
+                x = t.detach().double()
+                assert abs(float(x.sum()) - s1) <= 1e-5 * (1.0 + abs(s1)), (u, f)
+                assert abs(float((x * x).sum()) - s2) <= 1e-5 * (1.0 + abs(s2)), (u, f)
     runner = BatchedMarlRunner(env, net, buf, update_fn=update)
     stat = runner.train_process({})
+    assert n_batches[0] == len(want_fields) > 0
+    assert lock_steps == learner.a["update_lock_steps"].astype(int).tolist()
+    return learner, args, env, buf, runner, stat
+
+
+def test_reference_maddpg_learns_from_device_batches():
+    """The batches MADDPG's own optimisation steps learned from (changed weights, finite losses) when the recording was
+    made are the ones the runner delivers now (checked field by field in _run_on_device_batches); the learning itself
+    ran in the recording, not here. Also the runner's side of Model.train_process / evaluation: action range, transition
+    layout, done / last_step, hidden-state restarts, mean_train_* / mean_test_*."""
+    learner, args, env, buf, runner, stat = _run_on_device_batches("maddpg")
+    B, n, od, T = 5, 3, 7, 6
     assert runner.steps == T * B and buf.count == T
     # translate_action (utilities/util.py:123-132): every action the env saw lies inside [bias - scale, bias + scale]
     a = torch.stack(env.actions_seen)
@@ -117,56 +165,26 @@ def test_reference_maddpg_learns_from_device_batches(reference_on_path):
     assert float(lh.view(T, B, n, -1)[3].abs().max()) == 0.0 and float(lh.view(T, B, n, -1)[1].abs().max()) > 0.0
     # mean_train_* (model.py:243-261): info k is the constant k in the stand-in env
     assert abs(stat["mean_train_total_line_loss"] - 8.0) < 1e-12 and "mean_train_reward" in stat
-    assert updates and all(updates) and "mean_train_value_loss" in stat and np.isfinite(stat["mean_train_value_loss"])
     ev = runner.evaluation({}, num_eval_episodes=B)
     assert abs(ev["mean_test_destroy"] - 10.0) < 1e-12 and np.isfinite(ev["mean_test_reward"])
-
-
-def _reference_trainer(alg, n_agents, obs_dim, max_steps):
-    import yaml
-    from models.model_registry import Model as REGISTRY
-    from utilities.trainer import PGTrainer
-    d = yaml.safe_load(open(os.path.join(REF, "args", "default.yaml")))
-    d.update(yaml.safe_load(open(os.path.join(REF, "args", "alg_args", alg + ".yaml")))["alg_args"])
-    d.update(agent_num=n_agents, obs_size=obs_dim, action_dim=1, cuda=False, max_steps=max_steps, action_scale=0.8,
-             action_bias=0.0, batch_size=8)
-    args = namedtuple("Args", d.keys())(**d)
-    return args, PGTrainer(args, REGISTRY[alg], env=None, logger=None)
+    assert learner.done()
 
 
 @pytest.mark.parametrize("alg", ["iddpg", "maddpg", "matd3", "sqddpg", "facmaddpg", "mappo", "ippo", "coma"])
-def test_reference_algorithms_run_unchanged_on_device_batches(reference_on_path, alg):
+def test_reference_algorithms_run_unchanged_on_device_batches(alg):
     """Eight of the ten algorithms of the reference's registry (models/model_registry.py) collect experience through the
-    batched runner and run their own get_loss / optimiser steps on the device batches: deterministic and Gaussian
-    policies, twin critics (MATD3: value width 2), coalition sampling (SQDDPG: value width sample_size), a mixer
-    (FACMADDPG), PPO / COMA advantage code. Not covered, for reasons upstream: IAC (`self.cuda_` is never set:
-    models/iac.py:90 raises AttributeError with the reference's own env too) and MAAC (its value() returns a
+    batched runner, whose device batches their own get_loss / optimiser steps consumed when the recording was made:
+    deterministic and Gaussian policies, twin critics (MATD3: value width 2), coalition sampling (SQDDPG: value width
+    sample_size), a mixer (FACMADDPG), PPO / COMA advantage code. Not covered, for reasons upstream: IAC (`self.cuda_` is
+    never set: models/iac.py:90 raises AttributeError with the reference's own env too) and MAAC (its value() returns a
     concatenation that is not [batch, n, k]-shaped, models/maac.py:47-66)."""
-    from mapdn_b200.marl_runner import BatchedMarlRunner, DeviceTransitionBuffer, attach
-    B, n, od, T = 5, 3, 7, 6
-    args, trainer = _reference_trainer(alg, n, od, max_steps=T)
-    net = attach(trainer.behaviour_net)
-    env = FakeBatchedEnv(B, n, od, episode_limit=4)
-    buf = DeviceTransitionBuffer(32, B, n, od, act_dim=1, hid_dim=args.hid_size, device=env.device)
-    updates = []
-
-    def update(runner, stat):
-        if len(runner.buffer) >= 2 * args.batch_size:
-            batch = runner.buffer.get_batch(args.batch_size, n_windows=2)
-            w0 = [p.detach().clone() for p in trainer.behaviour_net.policy_dicts.parameters()]
-            trainer.value_transition_process(stat, batch)
-            trainer.policy_transition_process(stat, batch)
-            if args.mixer:
-                trainer.mixer_transition_process(stat, batch)
-            updates.append(any(not torch.equal(a, b) for a, b in zip(w0, trainer.behaviour_net.policy_dicts.parameters())))
-    runner = BatchedMarlRunner(env, net, buf, update_fn=update)
-    stat = runner.train_process({})
-    assert runner.steps == T * B and updates and all(updates)
-    assert np.isfinite(stat["mean_train_value_loss"]) and np.isfinite(stat["mean_train_policy_loss"])
+    learner, args, env, buf, runner, stat = _run_on_device_batches(alg)
+    B, T = 5, 6
+    assert runner.steps == T * B and np.isfinite(stat["mean_train_reward"])
     a = torch.stack(env.actions_seen)
     assert float(a.abs().max()) <= 0.8 + 1e-12                       # translate_action keeps the env's action range
     ev = runner.evaluation({}, num_eval_episodes=B)
-    assert np.isfinite(ev["mean_test_reward"])
+    assert np.isfinite(ev["mean_test_reward"]) and learner.done()
 
 
 class OracleBatchedEnv:
@@ -200,76 +218,45 @@ class OracleBatchedEnv:
 
 
 @pytest.mark.parametrize("alg", ["maddpg", "mappo"])
-def test_runner_collects_what_the_reference_train_process_collects(reference_on_path, alg, tmp_path):
-    """End to end against the reference's OWN loop: `Model.train_process` (models/model.py:197-263) drives the reference's
-    own env (oracle/ref_harness.py) with the reference's own learner; the batched runner drives the oracle-backed stand-in
-    with a copy of the same learner and the same torch seed. Every field of every transition (state, action, value,
-    next_value, reward, next_state, done, last_step, last_hid, hid) and the mean_train_* statistics agree."""
-    import copy
+def test_runner_collects_what_the_reference_train_process_collects(alg):
+    """End to end against the reference's OWN loop: `Model.train_process` (models/model.py:197-263) drove the reference's
+    own env (oracle/ref_harness.py) with the reference's own learner when the recording was made; the batched runner
+    drives the oracle-backed stand-in with the recorded learner. The learner's inputs, every field of every transition
+    (state, action, value, next_value, reward, next_state, done, last_step, last_hid, hid) and the mean_train_* /
+    mean_test_* statistics agree."""
     from mapdn_b200 import cases
     from mapdn_b200.marl_runner import BatchedMarlRunner, DeviceTransitionBuffer, attach
-    from oracle import ref_harness as H
     net, prof = cases.make_case("case33"), cases.make_profiles("case33", n_days=4)
     env_args = dict(voltage_barrier_type="bowl", action_scale=0.8, action_bias=0.0, seed=21)
-    H.write_reference_data(str(tmp_path), net, prof)
-    ref = H.ReferenceRun(str(tmp_path), net, env_args, env_id=0)             # episode 1 = the constructor's reset
-    T = 5
-    args, trainer = _reference_trainer(alg, net.n_sgen, ref.env.get_obs_size(), max_steps=T)
-    args = args._replace(replay_warmup=10 ** 9)                                # collection only: no update inside the loop
-    trainer.args = args
-    trainer.behaviour_net.args = args
-    model_copy = copy.deepcopy(trainer.behaviour_net)
-
-    class Hooked:                                                              # tells the harness which draws come next
-        def __init__(self, run):
-            self._r = run
-
-        def reset(self):
-            self._r.draws.begin_reset()
-            return self._r.env.reset()
-
-        def step(self, a):
-            self._r.draws.begin_step()
-            return self._r.env.step(a)
-
-        def __getattr__(self, k):
-            return getattr(self._r.env, k)
-
-    trainer.env = Hooked(ref)
-    torch.manual_seed(5)
-    stat_ref = {}
-    with ref._ctx():
-        trainer.behaviour_net.train_process(stat_ref, trainer)
-    trans = trainer.replay_buffer.buffer
-    assert len(trans) == T and trainer.steps == T
-
+    learner = RecordedLearner(f"{GOLDEN}/ref_learner_train_process_{alg}.npz", tol=1e-4)
+    g, args = learner.g, learner.args
+    T = args.max_steps
+    assert T == 5
     env = OracleBatchedEnv(net, prof, env_args, batch=1)
     env.reset()                                                                # episode 1, like the reference's constructor
-    buf = DeviceTransitionBuffer(T, 1, net.n_sgen, ref.env.get_obs_size(), act_dim=1, hid_dim=args.hid_size, device=env.device)
-    runner = BatchedMarlRunner(env, attach(model_copy), buf)
-    torch.manual_seed(5)
+    buf = DeviceTransitionBuffer(T, 1, net.n_sgen, env.obs_size, act_dim=1, hid_dim=args.hid_size, device=env.device)
+    runner = BatchedMarlRunner(env, attach(learner), buf)
     stat = runner.train_process({})
     st, ac, lp, v, nv, rw, ns, dn, ls, av, lh, h = buf.latest(T).unpacked()
+    ref = {k[6:]: learner.a[k] for k in learner.a if k.startswith("trans_")}
     tol = 2e-5                                                                 # the learner computes in fp32
-    for t, tr in enumerate(trans):
-        assert np.abs(np.array(tr.state) - st[t].numpy()).max() < tol and np.abs(np.array(tr.next_state) - ns[t].numpy()).max() < tol
-        assert np.abs(tr.action.reshape(-1) - ac[t].numpy().reshape(-1)).max() < tol
-        assert np.abs(tr.value.reshape(-1) - v[t].numpy().reshape(-1)).max() < 1e-4
-        assert np.abs(tr.next_value.reshape(-1) - nv[t].numpy().reshape(-1)).max() < 1e-4
-        assert np.abs(tr.reward - rw[t].numpy()).max() < tol
-        assert float(tr.done) == float(dn[t]) and float(tr.last_step) == float(ls[t])
-        assert np.abs(tr.last_hid.reshape(-1) - lh[t].numpy().reshape(-1)).max() < tol
-        assert np.abs(tr.hid.reshape(-1) - h[t].numpy().reshape(-1)).max() < tol
+    for t in range(T):
+        assert np.abs(ref["state"][t] - st[t].numpy()).max() < tol and np.abs(ref["next_state"][t] - ns[t].numpy()).max() < tol
+        assert np.abs(ref["action"][t].reshape(-1) - ac[t].numpy().reshape(-1)).max() < tol
+        assert np.abs(ref["value"][t].reshape(-1) - v[t].numpy().reshape(-1)).max() < 1e-4
+        assert np.abs(ref["next_value"][t].reshape(-1) - nv[t].numpy().reshape(-1)).max() < 1e-4
+        assert np.abs(ref["reward"][t] - rw[t].numpy()).max() < tol
+        assert float(ref["done"][t]) == float(dn[t]) and float(ref["last_step"][t]) == float(ls[t])
+        assert np.abs(ref["last_hid"][t].reshape(-1) - lh[t].numpy().reshape(-1)).max() < tol
+        assert np.abs(ref["hid"][t].reshape(-1) - h[t].numpy().reshape(-1)).max() < tol
+    stat_ref = json.loads(str(g["stat"]))
+    assert stat_ref
     for k, v_ref in stat_ref.items():
-        if k.startswith("mean_train_"):
-            assert abs(stat[k] - v_ref) < 1e-5, k
+        assert abs(stat[k] - v_ref) < 1e-5, k
     # Model.evaluation (models/model.py:265-302): greedy episodes, per-episode means averaged over the episodes
-    args = args._replace(num_eval_episodes=2)
-    trainer.args = trainer.behaviour_net.args = model_copy.args = args
-    ev_ref = {}
-    with ref._ctx():
-        trainer.behaviour_net.evaluation(ev_ref, trainer)
-    ev = runner.evaluation({}, num_eval_episodes=2)
-    assert len(ev_ref) == 12
+    ev_ref = json.loads(str(g["evaluation"]))
+    ev = runner.evaluation({}, num_eval_episodes=args.num_eval_episodes)
+    assert len(ev_ref) == 12 and args.num_eval_episodes == 2
     for k, v_ref in ev_ref.items():
         assert abs(ev[k] - v_ref) < 1e-5, k
+    assert learner.done()
