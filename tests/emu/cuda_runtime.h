@@ -79,9 +79,13 @@ static inline cudaError_t cudaMemsetAsync(void* d, int v, size_t n, cudaStream_t
 static inline cudaError_t cudaPointerGetAttributes(cudaPointerAttributes* a, const void* p) {   // every host buffer counts as pinned
   a->type = cudaMemoryTypeHost; a->device = 0; a->devicePointer = const_cast<void*>(p); a->hostPointer = const_cast<void*>(p); return cudaSuccess;
 }
-static inline cudaError_t cudaGetDeviceProperties(cudaDeviceProp* p, int) {                      // the B200 numbers the host code plans with
+// The B200 numbers the host code plans with. MAPDN_EMU_SMS overrides the SM count (read when a handle is created): with
+// one SM the planner picks the full-batch launch geometry (envs per CTA, shared-memory plan, several rounds of the
+// persistent loop per CTA) at batch sizes the emulation can run.
+static inline cudaError_t cudaGetDeviceProperties(cudaDeviceProp* p, int) {
   memset(p, 0, sizeof(*p)); snprintf(p->name, sizeof(p->name), "emulated B200");
-  p->multiProcessorCount = 148; p->sharedMemPerBlockOptin = 232448; p->sharedMemPerMultiprocessor = 233472; p->reservedSharedMemPerBlock = 1024;
+  const char* sms = getenv("MAPDN_EMU_SMS");
+  p->multiProcessorCount = sms ? std::max(1, atoi(sms)) : 148; p->sharedMemPerBlockOptin = 232448; p->sharedMemPerMultiprocessor = 233472; p->reservedSharedMemPerBlock = 1024;
   p->major = 10; p->minor = 0; p->totalGlobalMem = size_t(180) << 30; p->maxThreadsPerMultiProcessor = 2048; p->regsPerMultiprocessor = 65536;
   p->sharedMemPerBlock = 49152; p->warpSize = 32; return cudaSuccess;
 }

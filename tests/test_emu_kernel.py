@@ -99,13 +99,20 @@ def test_emulated_trajectory_matches_oracle(name, barrier, batch, lanes):
 def test_emulated_kernel_reproduces_the_reference_executed_fixtures(name):
     """The kernel source, on the CPU, against trajectories the reference's own env code produced
     (tests/golden/ref_env_*.npz, see tests/test_reference_golden.py)."""
+    replay_reference_fixture(name)
+
+
+def replay_reference_fixture(name, lead=0):
+    """Replays a reference-executed fixture on the emulated kernel. ``lead`` extra envs precede the fixture's envs in the
+    batch (``env_id_offset = -lead`` keeps their env ids, hence their random streams), which moves them to a later CTA
+    or a later round of the persistent loop. Returns the handle's dims."""
     g = np.load(S.fixture_path(ROOT, name))
     ops = [tuple(op) for op in json.loads(str(g["ops"]))]
     sc = S.SCENARIOS[name]
     net, prof = sc["build"]()
-    ids = sc["env_ids"]
+    ids = [lead + i for i in sc["env_ids"]]
     B = max(ids) + 1
-    env = EmuEnv(net, prof, sc["args"], batch=B)
+    env = EmuEnv(net, prof, sc["args"], batch=B, env_id_offset=-lead)
     t = n_reset = 0
     for k_op, op in enumerate(ops):
         if op[0] == "step":
@@ -133,6 +140,7 @@ def test_emulated_kernel_reproduces_the_reference_executed_fixtures(name):
         assert np.abs(env.obs[sel] - g["obs"][k_op, live][..., -env.dims["obs_dim"]:]).max() < TOL
         assert np.abs(env.get_state()[sel] - g["state"][k_op, live]).max() < 1e-8
     env.close()
+    return env.dims
 
 
 def _check_solve(net, lanes_list, B, rng, pl_hi, pv_hi):
