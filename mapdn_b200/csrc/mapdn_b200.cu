@@ -906,6 +906,16 @@ mapdn_status mapdn_create(const mapdn_net_desc* net, const mapdn_profile_desc* p
       const uint64_t sl_adj = pairs.count({std::min(b, slack), std::max(b, slack)}) ? 1 : 0;
       ndesc[i] = pa | (c0 << 16) | (c1 << 32) | (nx << 48) | (sl_adj << 63);
     }
+    {   // the slack injection sums over the slack's neighbours in this order: ascending bus index, so that the relabelling
+        // of section 2b cannot reorder the sum when the slack has several neighbours
+      std::vector<int> ks(sl_node.size());
+      for (size_t k = 0; k < ks.size(); ++k) ks[k] = static_cast<int>(k);
+      std::sort(ks.begin(), ks.end(), [&](int a, int b) { return order[sl_node[a]] < order[sl_node[b]]; });
+      std::vector<int> node2;
+      std::vector<double> y2;
+      for (int k : ks) { node2.push_back(sl_node[k]); y2.push_back(sl_y[2 * k]); y2.push_back(sl_y[2 * k + 1]); }
+      sl_node.swap(node2); sl_y.swap(y2);
+    }
     std::memcpy(hot.data() + hl.esched, esched.data(), 8 * esched.size());
     std::memcpy(hot.data() + hl.bsched, bsched.data(), 8 * bsched.size());
     std::memcpy(hot.data() + hl.lptr, lptr.data(), 2 * lptr.size());
@@ -972,8 +982,10 @@ mapdn_status mapdn_create(const mapdn_net_desc* net, const mapdn_profile_desc* p
     return pl;
   };
   bool cold_tables = false;
+  size_t least_smem = SIZE_MAX;          // the smallest footprint of any plan (one step of `unit` envs): reported when none fits
   {
     const Plan plans[4] = {make_plan(false, false), make_plan(false, true), make_plan(true, false), make_plan(true, true)};   // cheapest first
+    for (const Plan& pl : plans) if (pl.st2 > 0) least_smem = std::min(least_smem, smem_with(pl.cold, pl.st2, unit));
     const Plan* best = nullptr;
     for (const Plan& pl : plans) if (pl.ok && (!best || pl.rounds < best->rounds)) best = &pl;
     if (const char* ov = getenv("MAPDN_PLAN")) {             // tuning override: 0..3 = index into the list above
@@ -987,7 +999,8 @@ mapdn_status mapdn_create(const mapdn_net_desc* net, const mapdn_profile_desc* p
   auto smem_for = [&](int c) { return smem_with(cold_tables, stride2, c); };
   if (epb == 0 || smem_for(epb) > max_smem)
     return bail(fail(MAPDN_ERR_UNSUPPORTED, "network too large for the shared-memory resident solver (" +
-                                                std::to_string(smem_for(std::max(epb, unit))) + " B needed)"));
+                                                std::to_string(least_smem) + " B needed, " + std::to_string(max_smem) +
+                                                " B available)"));
   e->dense = meshed;
   e->G = G; e->threads = epb * G; e->epb = epb; e->smem = static_cast<int>(smem_for(epb));
   {   // helper warps (next profile rows + noise, concurrent with the Newton iteration): one per 256 Box-Muller pairs of a

@@ -168,9 +168,10 @@ class EmuEnv:
             self._chk(fn(self._h, _ptr(a), int(add_noise), _ptr(self.reward), _ptr(self.term), _ptr(self.info), _ptr(obs), None))
         return self.reward.copy(), self.term.copy(), self.info.copy(), obs
 
-    def droop(self, p_load, q_load, p_pv, s_rated, gain=0.1, tol=1e-4, max_ite=100):
+    def droop(self, p_load, q_load, p_pv, s_rated, gain=0.1, tol=1e-4, max_ite=100, q_max_manual=None):
         B, d = p_pv.shape[0], self.dims
-        ins = [np.ascontiguousarray(x, np.float64) for x in (p_load, q_load, p_pv, s_rated, s_rated)]
+        qmm = s_rated if q_max_manual is None else q_max_manual
+        ins = [np.ascontiguousarray(x, np.float64) for x in (p_load, q_load, p_pv, s_rated, qmm)]
         vm, q, loss, it = np.zeros((B, d["n_bus"])), np.zeros((B, d["n_sgen"])), np.zeros(B), np.zeros(B, np.int32)
         self._chk(lib().mapdn_droop(self._h, B, *[_ptr(x) for x in ins], float(gain), float(tol), int(max_ite), _ptr(vm), _ptr(q),
                                     _ptr(loss), _ptr(it), None))

@@ -223,9 +223,10 @@ def test_emulated_node_relabelling_changes_addresses_not_results(monkeypatch):
     e0.close(); e1.close()
 
 
-def _oracle_droop(net, pl, ql, pv, s_rated, max_ite=100, gain=0.1):
+def _oracle_droop(net, pl, ql, pv, s_rated, max_ite=100, gain=0.1, q_max_manual=None):
     """Literal restatement of reference traditional_control/pf_droop_matpower_all.m:121-152,196-231 (one instant)."""
     pf = PandapowerEquivalent(net)
+    qmm = s_rated if q_max_manual is None else q_max_manual
 
     def droop(p, s, v, qmm):
         q_max = min(np.sqrt(s * s - p * p), qmm)
@@ -241,7 +242,7 @@ def _oracle_droop(net, pl, ql, pv, s_rated, max_ite=100, gain=0.1):
         if np.linalg.norm(v_last - v) < 1e-4:
             break
         v_last = v
-        q_new = np.array([droop(pv[j], s_rated[j], v[j], s_rated[j]) for j in range(net.n_sgen)])
+        q_new = np.array([droop(pv[j], s_rated[j], v[j], qmm[j]) for j in range(net.n_sgen)])
         q_last = (1 - gain) * q_last + gain * q_new
     return res.vm_pu, q_last, res.pl_mw.sum(), i + 1
 
